@@ -1,6 +1,6 @@
 """bench.py — images/sec of the G+D training cycle (BASELINE.json metric) on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload resnet_cifar10]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload resnet_cifar10] [--dump-outputs DIR]
 
 A "step" is one ModularGAN cycle of `resnet_cifar10.gin` at batch 256 per GPU: disc_iters=5 D-updates +
 1 G-update on fresh synthetic images/z (unrolled semantics, reference gans/modular_gan.py:218-223), i.e.
@@ -224,6 +224,28 @@ def measure_cycle(workload, b, steps, warmup, mm, world, rank, eager=False, e2e=
           "launches_per_cycle": launches_per_cycle, "graph": graph, "losses": {"d": d_losses, "g": g_loss}}
 
 
+DUMP_VAR_BYTES = 60 * 10 ** 6      # keeps a dump, .npy headers and losses included, under 64 MB
+
+
+def dump_outputs(eng, out_dir):
+  """Writes what the timed cycle hands its caller after its last step, the losses of that step (d_losses.npy,
+  g_loss.npy) and the model variables it leaves behind (<variable name with '/' -> '.'>.npy), as float32 under out_dir.
+  When the variables exceed DUMP_VAR_BYTES in all, each is cut to a fixed, seeded sample of its flattened elements sized to
+  its share of that budget, so that runs of two builds with the same arguments can be compared file by file."""
+  d_losses, g_loss = eng.read_losses()
+  state = eng.state_numpy()
+  total = sum(v.nbytes for v in state.values())
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "d_losses.npy"), np.asarray(d_losses, np.float32))
+  np.save(os.path.join(out_dir, "g_loss.npy"), np.asarray([g_loss], np.float32))
+  for name, v in state.items():
+    a = np.asarray(v, np.float32)
+    if total > DUMP_VAR_BYTES:
+      keep = max(1, a.size * DUMP_VAR_BYTES // total)
+      a = a.ravel()[np.sort(np.random.RandomState(0).choice(a.size, keep, replace=False))]
+    np.save(os.path.join(out_dir, name.replace("/", ".") + ".npy"), a)
+
+
 def release(m):
   import gc
   import torch
@@ -324,6 +346,8 @@ def run_ours(args):
   m = measure_cycle(args.workload, b, args.steps, args.warmup, mm, world, rank, eager=args.eager, prof=prof)
   clocks = sampler.stop() if rank == 0 else None
   eng, ds, options, k = m["eng"], m["ds"], m["options"], m["k"]
+  if args.dump_outputs and rank == 0:
+    dump_outputs(eng, args.dump_outputs)
   ms_dev, ms_e2e = m["ms_dev"], m["ms_e2e"]
   images_per_step = b * (k + 1) * world
   value = images_per_step * args.steps / (ms_dev / 1e3)
@@ -540,6 +564,8 @@ def main():
   ap.add_argument("--dp-check", action="store_true", help="with --headline-only at N > 1: still run the in-run dp_equivalence check")
   ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU oracle leg (profiling runs only)")
   ap.add_argument("--eager", action="store_true", help="do not capture the cycle into a CUDA graph (profiling runs only)")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="after the timed steps, write the last step's losses and the model variables as float32 .npy under DIR")
   args = ap.parse_args()
   if args.impl == "reference":
     run_reference(args)

@@ -1,5 +1,8 @@
 """CPU tests of the host-side logic that needs no GPU: gin-compatible config surface, TF SAME padding
 arithmetic, dataset surface, metric math against the oracle and the reference's golden FID."""
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -9,8 +12,6 @@ from compare_gan_b200 import kernels as K
 from compare_gan_b200.metrics import fid_score, inception_score, kid_score
 from oracle import metrics as ometrics
 from oracle import tf_ops as T
-
-REF_CONFIGS = "/root/reference/example_configs"
 
 
 def test_same_padding_matches_oracle():
@@ -40,7 +41,6 @@ def test_gin_bindings_scopes_and_refs():
 
 
 def test_example_config_parses_and_binds():
-  import os
   from compare_gan_b200.gans import modular_gan  # noqa: F401
   from compare_gan_b200 import runner_lib  # noqa: F401
   gin.clear_config()
@@ -71,17 +71,15 @@ tf.train.AdamOptimizer.beta2 = 0.999
   assert opts["architecture"] == "resnet_cifar_arch" and opts["disc_iters"] == 5 and opts["lambda"] == 1
   assert opts["gan_class"] is modular_gan.ModularGAN
   assert gin.query_parameter("standardize_batch.decay") == 0.9
-  if os.path.isdir(REF_CONFIGS):   # in the build container: every shipped config must parse unmodified ...
-    from compare_gan_b200 import configs
-    for fn in sorted(os.listdir(REF_CONFIGS)):
-      if fn.endswith(".gin"):
-        gin.clear_config()
-        gin.parse_config(open(os.path.join(REF_CONFIGS, fn)).read())
-        assert runner_lib.get_options_dict()["gan_class"] is modular_gan.ModularGAN
-        from_file = gin.operative_config_str()
-        gin.clear_config()
-        gin.parse_config(configs.CONFIGS[fn[:-4]])     # ... and the restated copy must bind exactly the same values
-        assert gin.operative_config_str() == from_file, fn
+  # every example config the reference ships, restated in configs.py, must bind exactly the values the original file
+  # binds: the golden holds the operative config of each original example_configs/*.gin as parsed by gin_lite
+  from compare_gan_b200 import configs
+  golden = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "example_configs_operative.json")))
+  for name, from_file in sorted(golden.items()):
+    gin.clear_config()
+    gin.parse_config(configs.CONFIGS[name])
+    assert runner_lib.get_options_dict()["gan_class"] is modular_gan.ModularGAN
+    assert gin.operative_config_str() == from_file, name
   gin.clear_config()
 
 
