@@ -27,7 +27,7 @@ class ConvEpilogue(ctypes.Structure):
 
 CONV_RELU, CONV_ROUND_OUT, CONV_IN_TF32, CONV_IN2_TF32 = 1, 2, 4, 8
 ACT_ROUND_TF32 = 0x100
-OPT_TC_MT, OPT_LAST_PATH, OPT_TC_HALO, OPT_TC_PAIR, OPT_TC_EPI, OPT_TC_THIN = 1, 2, 3, 4, 5, 6
+OPT_TC_MT, OPT_LAST_PATH, OPT_TC_HALO, OPT_TC_THIN = 1, 2, 3, 6
 PATH_NAMES = {0: "simt_fp32", 1: "tcgen05_tf32", 2: "thin_fp32"}
 
 _SCALARS = {"int": ctypes.c_int, "int32_t": ctypes.c_int32, "int64_t": ctypes.c_int64,

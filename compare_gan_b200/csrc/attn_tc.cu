@@ -25,8 +25,6 @@
 //
 // Operands are consumed as TF32: callers pass tensors already rounded to the nearest TF32 value (cgan_round_tf32 or a
 // producer's ROUND_OUT epilogue); P and dS are rounded to nearest by the softmax warps.  Accumulation is fp32 in TMEM.
-#include <stdlib.h>
-
 #include "tc_common.cuh"
 
 namespace {
@@ -755,12 +753,11 @@ int cgan_attention_fwd(cgan_ctx* ctx, const float* q, const float* k, const floa
   if (!make_rows_map(&tq, q, dk, lq, batch, 128, false) || !make_rows_map(&tk, k, dk, lk, batch, 64, false) ||
       !make_rows_map(&tv, v, dv, lk, batch, 32, true))
     return cgan_fail(ctx, CGAN_ERR_CUDA, "%s: cuTensorMapEncodeTiled failed%s", "cgan_attention_fwd");
-  // Two CTAs per SM (default; 256 TMEM columns each) with rings as deep as half an SM's shared memory allows, or one CTA
-  // per SM with deeper rings (env CGAN_ATTN_CTAS=1).  Measured (profiles/r2_attention_*.txt): two resident CTAs overlap
-  // each other's per-tile dependency chains better than deeper prefetch in one.
-  static const int ctas = []() { const char* e = getenv("CGAN_ATTN_CTAS"); return (e && e[0] == '1') ? 1 : 2; }();
+  // Two CTAs per SM (256 TMEM columns each) with rings as deep as half an SM's shared memory allows.  Measured
+  // (profiles/r2_attention_*.txt): two resident CTAs overlap each other's per-tile dependency chains better than deeper
+  // prefetch in one CTA per SM (1.18 ms against 2.04 ms).
   const size_t v_stage = (size_t)p.vg * 8192, fixed = 16384 + 1280 + 1024;
-  const size_t budget = ctas == 2 ? (AT_SMEM_MAX - 2048) / 2 : AT_SMEM_MAX;
+  const size_t budget = (AT_SMEM_MAX - 2048) / 2;
   p.ns_a = AT_MAX_STAGES;
   p.ns_b = (int)((budget - fixed - (size_t)p.ns_a * 8192) / v_stage);
   if (p.ns_b > AT_MAX_STAGES) p.ns_b = AT_MAX_STAGES;

@@ -15,12 +15,9 @@ struct cgan_ctx {
   int math_mode;
   int64_t launches;
   int num_sms;
-  int tc_mt_max;       // tcgen05 kernels: max tiles per CTA sharing one operand tile (CGAN_OPT_TC_MT / env CGAN_TC_MT, default 2)
-  int tc_halo;         // 3x3 stride-1 tcgen05 convolutions use the halo variant (CGAN_OPT_TC_HALO / env CGAN_TC_HALO, default 1)
-  int tc_pair;         // tcgen05 convolutions run as CTA pairs sharing each weight tile (CGAN_OPT_TC_PAIR / env CGAN_TC_PAIR)
-  int tc_epi;          // coalescing (shared-memory transposed) epilogue of the tcgen05 convolutions (CGAN_OPT_TC_EPI / env CGAN_TC_EPI)
-  int tc_thin;         // image-side (<= 4 channel) convolutions through 32-wide patch tensors on tcgen05 (CGAN_OPT_TC_THIN / env CGAN_TC_THIN)
-  int tc_pair_mt;      // experiment knob: pixel tiles per CTA of the pair kernel (env CGAN_TC_PAIR_MT; 0 = automatic)
+  int tc_mt_max;       // tcgen05 kernels: max tiles per CTA sharing one operand tile (CGAN_OPT_TC_MT, default 2)
+  int tc_halo;         // 3x3 stride-1 tcgen05 convolutions use the halo variant (CGAN_OPT_TC_HALO, default 1)
+  int tc_thin;         // image-side (<= 4 channel) convolutions through 32-wide patch tensors on tcgen05 (CGAN_OPT_TC_THIN, default 1)
   int last_path;       // CGAN_PATH_* of the most recent contraction (cgan_ctx_get_option(CGAN_OPT_LAST_PATH))
   unsigned* counters;  // CGAN_NUM_COUNTERS zero-initialised tickets for single-launch two-stage reductions (norm.cu)
   void* p2p;           // peer-memory all-reduce state (p2p.cu), null until cgan_p2p_local_handle

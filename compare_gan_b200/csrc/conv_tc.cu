@@ -41,7 +41,6 @@ struct TcParams {
   int rows_used;                    // bw*bh*bni <= 128 pixel rows actually filled by the TMA box
   int img_n, img_h, img_w;          // extent of the pixel grid (tiles at the border hang over; those rows are not stored)
   int relu;                         // fused ReLU in the epilogue
-  int epi_stage;                    // 1: the epilogue transposes through shared memory for coalesced stores (tc_epilogue)
   int round_a;                      // 1: round the activation tiles to nearest TF32 in shared memory (operand not pre-rounded)
   int round_out;                    // 1: store TF32-rounded outputs (the consumer is another tensor-core contraction)
   float mask_leak;                  // with `mask`: out = ref > 0 ? v : mask_leak * v  ((leaky-)ReLU backward fused into a dgrad)
@@ -104,11 +103,11 @@ __device__ __forceinline__ void tc_tile_origin(const TcParams& p, int t, int& ow
 // one CTA per SM, ncu r2: 129 k wavefronts per SM) is bound by exactly that.  Each warp therefore transposes its
 // 32 x 32 chunk through a private 32 x 36-float staging area in the (by now idle) operand ring, after which a quarter
 // warp owns one row's 128 contiguous bytes: 4 wavefronts per store instruction, and the fused residual / mask reads
-// coalesce the same way.  `stg` = shared address of this warp's staging area (0: none, per-thread rows).
-constexpr int TC_EPI_ROW_BYTES = 36 * 4;                     // 32 columns + 16 B pad: 16-byte aligned, conflict-free v4 access
-constexpr int TC_EPI_WARP_BYTES = 32 * TC_EPI_ROW_BYTES;     // 4608 B per warp, 36 KB per CTA
+// coalesce the same way.  `stg` = shared address of this warp's staging area.
+constexpr int TC_STG_ROW_BYTES = 36 * 4;                     // 32 columns + 16 B pad: 16-byte aligned, conflict-free v4 access
+constexpr int TC_STG_WARP_BYTES = 32 * TC_STG_ROW_BYTES;     // 4608 B per warp, 36 KB per CTA (every operand ring holds >= 40 KB)
 
-__device__ __forceinline__ float4 tc_epilogue_math(const TcParams& p, float4 v, const float4 bv, long long off) {
+__device__ __forceinline__ float4 tc_out_math(const TcParams& p, float4 v, const float4 bv, long long off) {
   v.x += bv.x; v.y += bv.y; v.z += bv.z; v.w += bv.w;
   if (p.residual) {
     const float4 rv = *reinterpret_cast<const float4*>(p.residual + off);
@@ -124,14 +123,15 @@ __device__ __forceinline__ float4 tc_epilogue_math(const TcParams& p, float4 v, 
   return v;
 }
 
-__device__ __forceinline__ void tc_epilogue(const TcParams& p, uint32_t tmem_base, int tile0, int nt_here, int nb0, int warp,
-                                            int lane, long long out_base, uint32_t stg) {
+__device__ __forceinline__ void tc_store_tiles(const TcParams& p, uint32_t tmem_base, int tile0, int nt_here, int nb0,
+                                               int warp, int lane, long long out_base, uint32_t stg) {
   const int quarter = warp & 3;
   const int m = quarter * 32 + lane;
   const int wi = m % p.bw;
   const int hi = (m / p.bw) % p.bh;
   const int ni = m / (p.bw * p.bh);
   const int sub = lane >> 3, c4 = (lane & 7) * 4;       // transposed role: row (i*4 + sub) of the chunk, columns c4..c4+3
+  asm volatile("" : "+r"(stg));      // held in a register: ptxas would otherwise recompute it after every tcgen05.ld
   for (int tl = 0; tl < nt_here; ++tl) {
     int ow0, oh0, n0;
     tc_tile_origin(p, tile0 + tl, ow0, oh0, n0);
@@ -142,10 +142,8 @@ __device__ __forceinline__ void tc_epilogue(const TcParams& p, uint32_t tmem_bas
                            (long long)(ow0 + wi) * p.s_w + nb0;
     const uint32_t okmask = __ballot_sync(0xffffffffu, row_ok);
     long long roffs[8];
-    if (stg) {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) roffs[i] = __shfl_sync(0xffffffffu, roff, i * 4 + sub);
-    }
+    for (int i = 0; i < 8; ++i) roffs[i] = __shfl_sync(0xffffffffu, roff, i * 4 + sub);
     const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(tl * p.bn);
     // two warps share a lane quarter: the first takes the lower half of the 32-column chunks, the second the rest
     const int nchunks = p.bn / 32, csplit = (nchunks + 1) / 2;
@@ -154,10 +152,10 @@ __device__ __forceinline__ void tc_epilogue(const TcParams& p, uint32_t tmem_bas
       uint32_t r[32];
       tmem_ld32(taddr + (uint32_t)c0, r);
       const bool whole = nb0 + c0 + 32 <= p.cout && (p.cout & 3) == 0;      // warp-uniform
-      if (whole && stg) {
+      if (whole) {
 #pragma unroll
         for (int j = 0; j < 8; ++j)
-          sts128(stg + lane * TC_EPI_ROW_BYTES + j * 16,
+          sts128(stg + lane * TC_STG_ROW_BYTES + j * 16,
                  make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
                              __uint_as_float(r[4 * j + 3])));
         __syncwarp();
@@ -165,24 +163,13 @@ __device__ __forceinline__ void tc_epilogue(const TcParams& p, uint32_t tmem_bas
         if (p.bias) bv = *reinterpret_cast<const float4*>(p.bias + nb0 + c0 + c4);
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
-          const float4 v = lds128(stg + (i * 4 + sub) * TC_EPI_ROW_BYTES + c4 * 4);
+          const float4 v = lds128(stg + (i * 4 + sub) * TC_STG_ROW_BYTES + c4 * 4);
           if ((okmask >> (i * 4 + sub)) & 1u) {
             const long long off = roffs[i] + c0 + c4;
-            *reinterpret_cast<float4*>(p.out + off) = tc_epilogue_math(p, v, bv, off);
+            *reinterpret_cast<float4*>(p.out + off) = tc_out_math(p, v, bv, off);
           }
         }
         __syncwarp();
-      } else if (whole) {
-        if (row_ok) {
-#pragma unroll
-          for (int j = 0; j < 32; j += 4) {
-            const float4 v = make_float4(__uint_as_float(r[j]), __uint_as_float(r[j + 1]), __uint_as_float(r[j + 2]),
-                                         __uint_as_float(r[j + 3]));
-            float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (p.bias) bv = *reinterpret_cast<const float4*>(p.bias + nb0 + c0 + j);
-            *reinterpret_cast<float4*>(p.out + roff + c0 + j) = tc_epilogue_math(p, v, bv, roff + c0 + j);
-          }
-        }
       } else if (row_ok) {      // thin / padded tile (e.g. the 256->3 image conv): only the first `cout` columns exist
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
@@ -325,168 +312,14 @@ conv_tc_kernel(const __grid_constant__ AMaps tm_as, const __grid_constant__ CUte
     }
     mbar_wait(tmem_full_bar, 0);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    tc_epilogue(p, tmem_base, tile0, nt_here, nb0, warp, lane, p.ph_base[blockIdx.z],
-                p.epi_stage ? smem_u32(smem) + (warp - 2) * TC_EPI_WARP_BYTES : 0u);
+    tc_store_tiles(p, tmem_base, tile0, nt_here, nb0, warp, lane, p.ph_base[blockIdx.z],
+                   smem_u32(smem) + (warp - 2) * TC_STG_WARP_BYTES);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   }
   __syncthreads();
   if (warp == 1) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)p.tmem_cols) : "memory");
-  }
-}
-
-// ---- CTA-pair variant (cta_group::2) ------------------------------------------------------------------------------------
-// The per-tap kernel above is bound by the shared-memory pipe of the SM: per k-block and CTA the TMA engine writes
-// mt*16 KB + bn*128 B while the tensor core reads every operand byte again (the weight tile once per pixel tile) —
-// ~160 B/clk against 128 B/clk at bn = 256, ~220 B/clk at bn = 128.  Here two CTAs of a cluster (the two SMs of a TPC)
-// share every weight tile: each CTA loads and holds HALF of its rows, one tcgen05.mma.cta_group::2 of M = 256 multiplies
-// the pixel tiles of both CTAs with the whole tile, so both the TMA fill and the UMMA reads of the weight operand halve
-// per SM.  Protocol (see tc_common.cuh): both CTAs run a TMA producer whose loads complete on the LEADER's `full`
-// barrier (count 2: the leader's expect_tx arrive for the bytes of both CTAs + the peer's remote arrive), the leader's
-// MMA warp issues for both and commits `empty` / `tmem_full` with a multicast arrive to both CTAs, each CTA's epilogue
-// warps drain their own TMEM half.  Operands that still need rounding are rounded by each CTA's warps 2..9 in its own
-// shared memory; they arrive on the leader's `ready` barrier (count 2 x 8 warps).
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 2)
-conv_tc_pair_kernel(const __grid_constant__ AMaps tm_as, const __grid_constant__ CUtensorMap tm_b, const TcParams p) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int b_half_bytes = (p.bn / 2) * TC_BK * 4;
-  const int a_bytes = p.mt * TC_A_BYTES;
-  const int stage_bytes = a_bytes + b_half_bytes;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + p.stages * stage_bytes);
-  uint64_t* ready_bar = full_bar + p.stages;
-  uint64_t* empty_bar = ready_bar + p.stages;
-  uint64_t* tmem_full_bar = empty_bar + p.stages;
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tmem_full_bar + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const int tap0 = p.ph_tap0[blockIdx.z];
-  const int num_kb = (p.ph_tap0[blockIdx.z + 1] - tap0) * p.kchunks;
-  const int tile0 = blockIdx.x * p.mt;          // tiles beyond tiles_total are all-zero boxes whose rows are never stored
-  const int nb0 = blockIdx.y * p.bn;
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_as.m[0]) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_b) : "memory");
-  }
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < p.stages; ++s) {
-        mbar_init(&full_bar[s], p.round_a ? 1 : 2);      // pair mode: leader's expect_tx arrive + the peer's arrive
-        mbar_init(&ready_bar[s], 2 * TC_RWARPS);         // the rounding warps of both CTAs
-        mbar_init(&empty_bar[s], 1);
-      }
-      mbar_init(tmem_full_bar, 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr)), "r"((uint32_t)p.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  cluster_sync_all();                                    // barriers of both CTAs initialised before any remote arrive / TMA
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = *tmem_ptr;
-
-  if (warp == 0) {
-    // ===== TMA producer (both CTAs): own pixel tiles + own half of the weight tile, completing on the leader's barrier =====
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int kb = 0; kb < num_kb; ++kb) {
-        const int tl = kb / p.kchunks, kc = kb - tl * p.kchunks, tap = tap0 + tl;
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        uint8_t* sa = smem + stage * stage_bytes;
-        uint8_t* sb = sa + a_bytes;
-        const uint32_t own_bytes = (uint32_t)(p.mt * p.rows_used * TC_BK * 4 + b_half_bytes);
-        int ow0, oh0, n0;
-        if (p.round_a) {
-          // the operand is rounded in shared memory first: every CTA completes its loads on its OWN barrier, its rounding
-          // warps wait there and then arrive on the leader's `ready` barrier, which is what the MMA warp waits for
-          mbar_expect_tx(&full_bar[stage], own_bytes);
-          for (int i = 0; i < p.mt; ++i) {
-            tc_tile_origin(p, tile0 + i, ow0, oh0, n0);
-            tma_load_4d(sa + i * TC_A_BYTES, &tm_as.m[p.amap[tap]], &full_bar[stage], kc * TC_BK, ow0 + p.off_w[tap],
-                        oh0 + p.off_h[tap], n0);
-          }
-          tma_load_3d(sb, &tm_b, &full_bar[stage], kc * TC_BK, nb0 + (int)rank * (p.bn / 2), p.wtap[tap]);
-        } else {
-          if (leader) mbar_expect_tx(&full_bar[stage], 2 * own_bytes);
-          else mbar_arrive_cluster(&full_bar[stage], 0);
-          for (int i = 0; i < p.mt; ++i) {
-            tc_tile_origin(p, tile0 + i, ow0, oh0, n0);
-            tma_load_4d_pair(sa + i * TC_A_BYTES, &tm_as.m[p.amap[tap]], &full_bar[stage], kc * TC_BK, ow0 + p.off_w[tap],
-                             oh0 + p.off_h[tap], n0);
-          }
-          tma_load_3d_pair(sb, &tm_b, &full_bar[stage], kc * TC_BK, nb0 + (int)rank * (p.bn / 2), p.wtap[tap]);
-        }
-        if (++stage == p.stages) { stage = 0; phase ^= 1; }
-      }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer: the leader only, for both CTAs =====
-    if (leader) {
-      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(p.bn >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int kb = 0; kb < num_kb; ++kb) {
-        mbar_wait(p.round_a ? &ready_bar[stage] : &full_bar[stage], phase);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        if (lane == 0) {
-          const uint32_t a_addr = smem_u32(smem + stage * stage_bytes);
-          const uint32_t b_addr = a_addr + a_bytes;
-          for (int i = 0; i < p.mt; ++i) {
-#pragma unroll
-            for (int k = 0; k < TC_BK / 8; ++k)
-              umma_tf32_pair(tmem_base + (uint32_t)(i * p.bn), make_desc(a_addr + i * TC_A_BYTES + k * 32), make_desc(b_addr + k * 32),
-                             idesc, (kb | k) ? 1u : 0u);
-          }
-          umma_commit_pair(&empty_bar[stage]);
-          if (kb == num_kb - 1) umma_commit_pair(tmem_full_bar);
-        }
-        __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1; }
-      }
-    }
-  } else {
-    // ===== warps 2..9: round the own A tiles (operand not pre-rounded), then the epilogue of the own tiles =====
-    const int q = threadIdx.x - 64;
-    if (p.round_a) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int kb = 0; kb < num_kb; ++kb) {
-        mbar_wait(&full_bar[stage], phase);              // this CTA's own loads (local completion in rounding mode)
-        uint32_t a4 = smem_u32(smem + stage * stage_bytes) + q * 16;
-        for (int tl = 0; tl < p.mt; ++tl, a4 += TC_A_BYTES) {
-          float4 v[TC_A_BYTES / 16 / (32 * TC_RWARPS)];
-#pragma unroll
-          for (int i = 0; i < TC_A_BYTES / 16 / (32 * TC_RWARPS); ++i) v[i] = lds128(a4 + i * (512 * TC_RWARPS));
-#pragma unroll
-          for (int i = 0; i < TC_A_BYTES / 16 / (32 * TC_RWARPS); ++i) {
-            v[i].x = rna_tf32(v[i].x); v[i].y = rna_tf32(v[i].y); v[i].z = rna_tf32(v[i].z); v[i].w = rna_tf32(v[i].w);
-            sts128(a4 + i * (512 * TC_RWARPS), v[i]);
-          }
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(&ready_bar[stage], 0);
-        if (++stage == p.stages) { stage = 0; phase ^= 1; }
-      }
-    }
-    mbar_wait(tmem_full_bar, 0);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    tc_epilogue(p, tmem_base, tile0, p.mt, nb0, warp, lane, p.ph_base[blockIdx.z],
-                p.epi_stage ? smem_u32(smem) + (warp - 2) * TC_EPI_WARP_BYTES : 0u);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  }
-  __syncthreads();
-  cluster_sync_all();                                    // the peer's TMEM / barriers stay alive until both CTAs are done
-  if (warp == 1) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)p.tmem_cols) : "memory");
   }
 }
 
@@ -629,8 +462,7 @@ conv_tc_halo_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
     }
     mbar_wait(tmem_full_bar, 0);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    tc_epilogue(p, tmem_base, tile0, nt_here, nb0, warp, lane, p.base,
-                p.epi_stage ? smem_u32(smem) + (warp - 2) * TC_EPI_WARP_BYTES : 0u);
+    tc_store_tiles(p, tmem_base, tile0, nt_here, nb0, warp, lane, p.base, smem_u32(smem) + (warp - 2) * TC_STG_WARP_BYTES);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   }
   __syncthreads();
@@ -757,7 +589,6 @@ int cgan_conv_tc(cgan_ctx* ctx, const float* in, int nviews, const long long* vi
   p.rows_used = p.bw * p.bh * p.bni;
   p.img_n = n; p.img_h = gh; p.img_w = gw;
   p.relu = relu;
-  p.epi_stage = ctx->tc_epi;          // every ring below holds >= 40 KB >= 8 warps x TC_EPI_WARP_BYTES
   p.round_a = (ex && ex->a_prerounded) ? 0 : 1;
   if (ex) {
     p.round_out = ex->round_out; p.residual = ex->residual; p.mask = ex->mask; p.mask_leak = ex->mask_leak;
@@ -903,60 +734,6 @@ int cgan_conv_tc(cgan_ctx* ctx, const float* in, int nviews, const long long* vi
     CUresult r = enc(&tm_b, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, wt, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return cgan_fail(ctx, CGAN_ERR_CUDA, "%s: cuTensorMapEncodeTiled(B) failed%s", "cgan_conv_tc");
-  }
-  // ---- CTA-pair variant: two SMs share every weight tile (cta_group::2) --------------------------------------------------
-  if (ctx->tc_pair && wimg_stride == 0 && ncols_pad % 64 == 0) {
-    const long long tiles_total = (long long)p.tiles_w * p.tiles_h * tiles_n;
-    TcParams q = p;
-    q.bn = tc_pick_bn(ncols_pad);                 // widest column tile: the pair is about weight-tile reuse
-    const int ncol_tiles = ncols_pad / q.bn;
-    q.mt = 1;
-    for (int m = 4; m >= 2; --m)
-      if (m * q.bn <= 512 && tiles_total * ncol_tiles * q.nphases >= 2ll * m * ctx->num_sms) { q.mt = m; break; }
-    if (ctx->tc_mt_max < 2) q.mt = 1;
-    if (ctx->tc_pair_mt > 0 && ctx->tc_pair_mt * q.bn <= 512) q.mt = ctx->tc_pair_mt;       // experiment knob (CGAN_TC_PAIR_MT)
-    const long long groups = (tiles_total + q.mt - 1) / q.mt;
-    if (q.bn % 32 == 0 && q.bn >= 64 && groups * ncol_tiles * q.nphases >= ctx->num_sms) {
-      const size_t stage_bytes = (size_t)q.mt * TC_A_BYTES + (size_t)(q.bn / 2) * TC_BK * 4;
-      // two CTA pairs per SM pair when the accumulators take at most half of the TMEM: one pair's epilogue then overlaps
-      // the other's main loop
-      const bool two_per_sm = q.mt * q.bn <= 256;
-      q.stages = (int)(((two_per_sm ? 113 : 227) * 1024 - 1024 - 512) / stage_bytes);
-      if (q.stages > 6) q.stages = 6;
-      if (q.stages >= 2) {
-        q.tiles_total = (int)tiles_total;
-        q.tmem_cols = 32;
-        while (q.tmem_cols < q.mt * q.bn) q.tmem_cols *= 2;
-        AMaps tma;
-        memset(&tma, 0, sizeof(tma));
-        for (int v = 0; v < 4; ++v) {
-          int vv = v < nviews ? v : 0;
-          int vh = h, vw = w;
-          if (nviews == 4 && view_phase_of) { vh = (view_phase_of[0] - (vv >> 1) + 1) / 2; vw = (view_phase_of[1] - (vv & 1) + 1) / 2; }
-          if (vh < 1 || vw < 1) { vh = h; vw = w; vv = 0; }
-          if (!make_act_map(&tma.m[v], in + view_off[vv], kdim, vw, vh, n, in_sw, in_sh, in_sn, q.bw, q.bh, q.bni))
-            return cgan_fail(ctx, CGAN_ERR_CUDA, "%s: cuTensorMapEncodeTiled(A) failed%s", "cgan_conv_tc");
-        }
-        CUtensorMap tmb;
-        cuuint64_t dims[3] = {(cuuint64_t)kdim_pad, (cuuint64_t)ncols_pad, (cuuint64_t)taps_total};
-        cuuint64_t strides[2] = {(cuuint64_t)kdim_pad * 4, (cuuint64_t)ncols_pad * kdim_pad * 4};
-        cuuint32_t box[3] = {TC_BK, (cuuint32_t)(q.bn / 2), 1};
-        cuuint32_t es[3] = {1, 1, 1};
-        if (enc(&tmb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, wt, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-          return cgan_fail(ctx, CGAN_ERR_CUDA, "%s: cuTensorMapEncodeTiled(B half) failed%s", "cgan_conv_tc");
-        size_t smem = (size_t)q.stages * stage_bytes + 1024 + 512;
-        static bool pair_attr_set = false;
-        if (!pair_attr_set) {
-          CGAN_CUDA(ctx, cudaFuncSetAttribute(conv_tc_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-          pair_attr_set = true;
-        }
-        dim3 grid((unsigned)((groups + 1) / 2 * 2), (unsigned)ncol_tiles, (unsigned)q.nphases);
-        conv_tc_pair_kernel<<<grid, TC_THREADS, smem, ctx->stream>>>(tma, tmb, q);
-        CGAN_LAUNCHED(ctx);
-        return CGAN_OK;
-      }
-    }
   }
 
   // Two CTAs per SM (each owns 256 of the 512 TMEM columns): one CTA's epilogue and prologue overlap the other's main

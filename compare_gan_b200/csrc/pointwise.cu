@@ -25,16 +25,8 @@ int cgan_ctx_create(cgan_ctx** out, int device) {
   if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) { delete c; return CGAN_ERR_CUDA; }
   c->num_sms = prop.multiProcessorCount;
   c->tc_mt_max = 2;
-  if (const char* e = getenv("CGAN_TC_MT")) c->tc_mt_max = atoi(e) >= 2 ? 2 : 1;
-  c->tc_pair = 0;
-  if (const char* e = getenv("CGAN_TC_PAIR")) c->tc_pair = atoi(e) ? 1 : 0;
-  if (const char* e = getenv("CGAN_TC_PAIR_MT")) c->tc_pair_mt = atoi(e);
-  c->tc_epi = 1;
-  if (const char* e = getenv("CGAN_TC_EPI")) c->tc_epi = atoi(e) ? 1 : 0;
   c->tc_halo = 1;
-  if (const char* e = getenv("CGAN_TC_HALO")) c->tc_halo = atoi(e) ? 1 : 0;
   c->tc_thin = 1;
-  if (const char* e = getenv("CGAN_TC_THIN")) c->tc_thin = atoi(e) ? 1 : 0;
   c->stream = 0;
   if (cudaMalloc(reinterpret_cast<void**>(&c->counters), CGAN_NUM_COUNTERS * sizeof(unsigned)) != cudaSuccess ||
       cudaMemset(c->counters, 0, CGAN_NUM_COUNTERS * sizeof(unsigned)) != cudaSuccess) {
@@ -79,14 +71,6 @@ int cgan_ctx_set_option(cgan_ctx* ctx, int key, int64_t value) {
       CGAN_REQUIRE(ctx, value == 1 || value == 2, "CGAN_OPT_TC_MT must be 1 or 2");
       ctx->tc_mt_max = (int)value;
       return CGAN_OK;
-    case CGAN_OPT_TC_PAIR:
-      CGAN_REQUIRE(ctx, value == 0 || value == 1, "CGAN_OPT_TC_PAIR must be 0 or 1");
-      ctx->tc_pair = (int)value;
-      return CGAN_OK;
-    case CGAN_OPT_TC_EPI:
-      CGAN_REQUIRE(ctx, value == 0 || value == 1, "CGAN_OPT_TC_EPI must be 0 or 1");
-      ctx->tc_epi = (int)value;
-      return CGAN_OK;
     case CGAN_OPT_TC_HALO:
       CGAN_REQUIRE(ctx, value >= 0 && value <= 2, "CGAN_OPT_TC_HALO must be 0, 1 or 2");
       ctx->tc_halo = (int)value;
@@ -107,8 +91,6 @@ int cgan_ctx_get_option(cgan_ctx* ctx, int key, int64_t* host_value) {
     case CGAN_OPT_TC_MT: *host_value = ctx->tc_mt_max; return CGAN_OK;
     case CGAN_OPT_LAST_PATH: *host_value = ctx->last_path; return CGAN_OK;
     case CGAN_OPT_TC_HALO: *host_value = ctx->tc_halo; return CGAN_OK;
-    case CGAN_OPT_TC_PAIR: *host_value = ctx->tc_pair; return CGAN_OK;
-    case CGAN_OPT_TC_EPI: *host_value = ctx->tc_epi; return CGAN_OK;
     case CGAN_OPT_TC_THIN: *host_value = ctx->tc_thin; return CGAN_OK;
     default:
       return cgan_fail(ctx, CGAN_ERR_ARG, "%s: unknown option%s", "cgan_ctx_get_option");

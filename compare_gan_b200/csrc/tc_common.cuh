@@ -53,52 +53,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-// ---- CTA-pair (cta_group::2) forms ------------------------------------------------------------------------------------
-// Two CTAs of one cluster (the two SMs of a TPC) execute ONE tcgen05.mma of M = 256: rows 0..127 come from the leader's
-// shared memory / accumulate in the leader's TMEM, rows 128..255 in the peer's; each CTA holds HALF of the B tile (N/2
-// rows).  Only the leader issues MMAs; TMA loads of both CTAs complete on the LEADER's mbarrier (its shared::cluster
-// address is the local one with the peer bit 24 cleared); tcgen05.commit multicasts its arrival to both CTAs.
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive (count 1) on the mbarrier at the same shared-memory offset in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t cta) {
-  uint32_t remote;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_u32(bar)), "r"(cta));
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_pair(void* dst, const CUtensorMap* map, uint64_t* leader_bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(leader_bar) & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_load_3d_pair(void* dst, const CUtensorMap* map, uint64_t* leader_bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(leader_bar) & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void umma_tf32_pair(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-      "}\n" ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
-}
-// arrival on the barrier at this offset in BOTH CTAs of the pair once the MMAs issued so far have retired
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
-}
-
 // explicit shared-space 128-bit accesses: a pointer carved out of the dynamic smem buffer compiles to GENERIC LD/ST
 // (ncu source page: LD.E.128 / ST.E.128 with long-scoreboard stalls); these are LDS.128 / STS.128
 __device__ __forceinline__ float4 lds128(uint32_t addr) {

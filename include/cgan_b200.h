@@ -45,17 +45,12 @@ int64_t cgan_launch_count(cgan_ctx* ctx);
  *   CGAN_OPT_TC_HALO    (set/get) 3x3 stride-1 tcgen05 convolutions fetch one (rows+2)-row activation box per kernel column
  *                       instead of one box per tap: 0 never, 1 where it measured faster (operand rounded in the kernel,
  *                       >= 256 output channels; default), 2 wherever the geometry allows.
- *   CGAN_OPT_TC_PAIR    (set/get) 1: tcgen05 convolutions run as CTA pairs (cta_group::2, M = 256) sharing each weight tile.
- *   CGAN_OPT_TC_EPI     (set/get) 1 (default): the tcgen05 convolution epilogue transposes each 32 x 32 accumulator chunk through
- *                       shared memory so that stores (and the fused residual / mask reads) cover whole 128-byte lines;
- *                       0: every thread stores its own row (the round-1 epilogue; results are bit-identical).
  *   CGAN_OPT_TC_THIN    (set/get) 1 (default): in math_mode 1 the image-side convolutions (<= 4 input or <= 4 output channels,
  *                       kh*kw*channels <= 32: every discriminator's first and every generator's last convolution, Inception's
  *                       stem) run as ONE 32-wide GEMM on the tcgen05 kernels over a [pixels, 32] patch tensor (csrc/thin_tc.cu),
  *                       TF32 operands like every other tensor-core contraction; 0: the exact-fp32 streaming kernels (thin.cu).
  *   CGAN_OPT_LAST_PATH  (get) CGAN_PATH_* taken by the most recent conv2d_fwd / dgrad / wgrad / gemm_batched call. */
-enum { CGAN_OPT_TC_MT = 1, CGAN_OPT_LAST_PATH = 2, CGAN_OPT_TC_HALO = 3, CGAN_OPT_TC_PAIR = 4, CGAN_OPT_TC_EPI = 5,
-       CGAN_OPT_TC_THIN = 6 };
+enum { CGAN_OPT_TC_MT = 1, CGAN_OPT_LAST_PATH = 2, CGAN_OPT_TC_HALO = 3, CGAN_OPT_TC_THIN = 6 };
 enum { CGAN_PATH_SIMT_FP32 = 0, CGAN_PATH_TCGEN05_TF32 = 1, CGAN_PATH_THIN_FP32 = 2 };
 int cgan_ctx_set_option(cgan_ctx* ctx, int key, int64_t value);
 int cgan_ctx_get_option(cgan_ctx* ctx, int key, int64_t* host_value);

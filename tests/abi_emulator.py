@@ -73,10 +73,10 @@ class EmulatedLib(object):
     return self.launches
 
   def get_option(self, key):
-    return {1: 2, 2: self.last_path, 3: 1, 4: 0, 5: 1, 6: 1}[key]
+    return {1: 2, 2: self.last_path, 3: 1, 6: 1}[key]
 
   def set_option(self, key, value):
-    assert (key == 1 and value in (1, 2)) or (key == 3 and value in (0, 1, 2)) or (key in (4, 5, 6) and value in (0, 1))
+    assert (key == 1 and value in (1, 2)) or (key == 3 and value in (0, 1, 2)) or (key == 6 and value in (0, 1))
 
   def call(self, name, *args):
     self.launches += 1
